@@ -7,9 +7,12 @@ synthetic random Connect-Four positions), every new node evaluated by the 7-bloc
   e2e   : the same through the host-buffer seam az_mcts_explore (H2D roots + eta, run, D2H N/W/P inside the timed region)
 Trees are sharded over ranks with no data-path collective (weak scaling: 4096 trees per GPU).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   --impl reference : the reference's algorithm on the host CPU cores (oracle port + torch-CPU fp32 network),
                      rank 0 only, on a bounded sample of the same workload.
+  --dump-outputs   : after the timed steps, write the root statistics N, W, P [trees, 7] of the last device-resident step
+                     and e2e_N, e2e_W, e2e_P of the last end-to-end step as DIR/<name>.npy (float64, P float32; suffix
+                     _rank<r> with several ranks).  The inputs are seeded, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -137,6 +140,21 @@ def make_eta(_unused, roots, A, seed):
     return eta
 
 
+DUMP_BYTES = 60 * 10**6   # all ranks together, .npy headers aside: a dump stays under 64 MB at any --trees
+
+
+def dump_outputs(d, arrays, rank, world):
+    """Writes `arrays` (one row per tree) as d/<name>.npy in float64 (float32 arrays stay float32).  Above this rank's share
+    of DUMP_BYTES every array keeps the same fixed, seeded sample of rows (in tree order)."""
+    arrays = {k: np.asarray(v, np.float32 if v.dtype == np.float32 else np.float64) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    keep = min(n, DUMP_BYTES // world // sum(a[0].nbytes for a in arrays.values()))
+    rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False)) if keep < n else slice(None)
+    os.makedirs(d, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(d, k + ("_rank%d" % rank if world > 1 else "") + ".npy"), a[rows])
+
+
 def product_config(S, nsims, blocks, oracle_net, world):
     """The `config` object of a bench line (both arms print the same one for the same workload)."""
     return {"workload": "connect-four: %d concurrent game trees per GPU x %d sims/move, %s, synthetic random positions (0-30 plies), fresh trees per step"
@@ -238,7 +256,12 @@ def main():
     ap.add_argument("--no-selfplay", action="store_true", help="skip the full self-play leg (games/s)")
     ap.add_argument("--cpu-threads", type=int, default=0, help="threads of the CPU reference arm (0 = min(cores, 16): torch-CPU conv throughput peaks there on the 128-core box)")
     ap.add_argument("--oracle-net", default=None, choices=[None, "uniform", "synth"], help="tree-only figure: built-in oracle instead of the ResNet")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the root statistics of the last timed steps as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -287,9 +310,9 @@ def main():
     def step_e2e():
         env.reset()
         t0 = time.perf_counter()
-        N, W, P = env.explore(roots, nsims, eta)   # H2D roots+eta, 600 sims, D2H N/W/P
+        NWP = env.explore(roots, nsims, eta)   # H2D roots+eta, 600 sims, D2H N/W/P
         dt = time.perf_counter() - t0
-        return dt, env.last_timing()["expansions"], N
+        return dt, env.last_timing()["expansions"], NWP
 
     env.set_roots(roots, eta)
     for _ in range(args.warmup):
@@ -308,6 +331,8 @@ def main():
         barrier()
         t_wall = time.perf_counter() - t_wall
     launches = ctx.num_launches - l0
+    if args.dump_outputs:
+        resident_NWP = env.root_stats()   # the last timed step's trees, before the passes below rebuild them
     # ---- roofline pass: the same steps again with CUDA events around the tower launches (events on the library's own
     #      stream; recording them per launch disables graph replay, hence a separate pass) ----
     prof = None
@@ -339,10 +364,12 @@ def main():
     barrier()
     e_dt, e_ex = 0.0, 0
     for _ in range(args.steps):
-        d, e, N = step_e2e()
+        d, e, e2e_NWP = step_e2e()
         e_dt += d
         e_ex += e
     barrier()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(("N", "W", "P", "e2e_N", "e2e_W", "e2e_P"), resident_NWP + e2e_NWP)), rank, world)
     sims = args.steps * S * nsims
     # ---- full self-play (games/s): simulate() with the shipped Connect-Four MctsParams, one game per slot ----
     sp_out = None
