@@ -2,22 +2,27 @@
 // evaluate_batch: src/networks/flux.jl:127-132, src/networks/network.jl:264-271,308-315, and the Flux layers of
 // src/networks/architectures/resnet.jl:53-92 and simplenet.jl:37-64).
 //
-// Data layout in HBM.  Activations are fp16 "padded NHWC" rows of F=128 channels:
-//     row(board b, col x, row y) = b*BS + y*(W+1) + x,   BS = (W+1)*(H+1)      (Connect-Four: BS = 56)
-// with column x = W and row y = H kept at ZERO, so that the 3x3 "same" convolution becomes nine row-shifted GEMMs
-//     out[p, co] = sum_{tap} sum_{ci} act[p + off(tap), ci] * Wt[co, tap*F + ci],   off = dy*(W+1) + dx
-// and each tap's A operand is ONE TMA box of consecutive rows (out-of-range rows are zero-filled by TMA).
+// Activation layouts in HBM (fp16 rows of F = 128 channels, chosen once per network in ResNetImpl::init):
+//   * DENSE, for the Connect-Four tower (7 x 6 boards, num_blocks > 0): row(board b, col x, row y) = b*W*H + y*W + x.
+//     The tower kernels see it as a 4-D tensor (channel, x, y, board); the "same" padding of the 3x3 convolution is the
+//     zero fill of TMA boxes that start at x = -1 (see az_k_conv_yrow).
+//   * PADDED NHWC, for every other geometry: row(b, x, y) = b*BS + y*(W+1) + x, BS = (W+1)*(H+1), with column x = W and
+//     row y = H kept at ZERO, so that the 3x3 "same" convolution becomes nine row-shifted GEMMs
+//         out[p, co] = sum_{tap} sum_{ci} act[p + off(tap), ci] * Wt[co, tap*F + ci],   off = dy*(W+1) + dx
+//     and each tap's A operand is ONE TMA box of consecutive rows (out-of-range rows are zero-filled by TMA).
 //
-// Kernels in this file:
-//   az_k_im2col          leaf states -> 64-wide fp16 im2col rows of the first conv (game's vectorize_state on device)
-//   az_k_gemm_tc<BN,EPI> generic warp-specialised tcgen05 implicit GEMM (TMA producer warp -> 6-stage SWIZZLE_128B smem
-//                        ring -> one elected lane issues tcgen05.mma M=128,N=BN,K=16 fp16->fp32 into double-buffered TMEM
-//                        -> 4 epilogue warps).  Used for the stem conv, the towers of non-Connect-Four geometries, the
-//                        heads' 1x1 convs (N=64) and the value / policy dense layers (plain K-major GEMMs).
-//   az_k_conv_c4_2sm<EPI> Connect-Four tower conv: 2-CTA cluster, cta_group::2 MMA, resident half-N weights, 3 dx-shifted
-//                        A copies reused by the dy taps, coalesced epilogue with the fp32 residual stream.
-//   az_k_finalize        softmax + legal-action mask + renormalisation, tanh value.
-//   az_k_simplenet       fused fp32 MLP (SimpleNet).
+// Kernels in this file (tcgen05 MMAs fed by TMA, fp16 operands, fp32 accumulators in TMEM):
+//   az_k_stem<G>          leaf states -> first conv: the im2col tile is built in shared memory, one launch (both layouts)
+//   az_k_tower_yrow       Connect-Four tower, ALL conv layers in one persistent launch: 2-CTA clusters (cta_group::2),
+//                         resident weights, skip connection added on the tensor core from an fp16 + e4m3 residual stream
+//   az_k_conv_yrow<EPI>   the same tower one conv layer per launch (AZ_TOWER=layer): the reference the persistent kernel
+//                         is tested against bit for bit (with AZ_LO=16)
+//   az_k_gemm_tc<BN,EPI>  generic warp-specialised implicit GEMM over the padded layout: the tower of every other
+//                         geometry (tic-tac-toe, mancala, grid world), fp32 residual stream
+//   az_k_head_conv        both heads' 1x1 convs as one N = 64 GEMM
+//   az_k_heads_dense<G>   value dense + tanh and policy dense + softmax + legal-action mask, one launch
+//   az_k_simplenet<G,NB>  fused fp32 MLP (SimpleNet)
+//   az_k_fold_conv / az_k_fold_dense   parameter blob -> the kernels' weight layouts
 // BatchNorm (test mode, eps = 1e-5) is folded into the conv / dense weights and biases when the blob is loaded.
 #include <cuda.h>
 #include <cuda_fp16.h>
@@ -139,13 +144,14 @@ __device__ __forceinline__ uint64_t umma_desc_interleave(uint32_t saddr, uint32_
 }
 
 // ------------------------------------------------------------------------------------------------
-// tcgen05 implicit-GEMM kernel: tower convs, the heads' 1x1 convs and the value head's dense layer all run here
+// generic tcgen05 implicit-GEMM kernel (TMA producer warp -> 6-stage SWIZZLE_128B smem ring -> one elected lane issues
+// tcgen05.mma M=128,N=BN,K=16 into double-buffered TMEM -> 4 epilogue warps): the tower convs of the padded layout
 // ------------------------------------------------------------------------------------------------
 namespace tc {
 constexpr int BM = 128, BK = 64, STAGES = 6, F = 128;
 constexpr int A_BYTES = BM * BK * 2;
 constexpr int NUM_THREADS = 192;
-enum { EPI_CONV1 = 0, EPI_CONV2 = 1, EPI_HEAD = 2, EPI_DENSE = 3 };
+enum { EPI_CONV1 = 0, EPI_CONV2 = 1 };
 template <int BN>
 struct Smem {
   uint8_t a[STAGES][A_BYTES];
@@ -170,24 +176,23 @@ struct ConvGeom {
 struct GemmArgs {
   const int32_t* n_boards;
   ConvGeom g;
-  int kblocks;       // number of 64-wide K blocks
-  int gemm_k;        // 0: A coords = ((kb&1)*64, row + off[kb>>1]) (shifted-row conv);  1: A coords = (kb*64, row) (plain GEMM)
-  int rows_per_board;  // rows of the M dimension per board: board_rows (conv/head) or 1 (dense)
+  int kblocks;       // number of 64-wide K blocks: A coords = ((kb&1)*64, row + off[kb>>1]) (shifted-row conv)
+  int rows_per_board;  // rows of the M dimension per board (board_rows)
   int alloc_rows;
-  int no_relu;           // EPI_DENSE: 1 = plain affine output (policy logits)
-  int debug;             // timing experiments only (AZ_TOWER_DEBUG bitmask): 4 = no epilogue global I/O
   const float* bias;
   const float* resid32;  // EPI_CONV2
   int lo8;               // persistent tower: 1 = low-order residual part stored as e4m3 bytes (XL8), 0 = fp16 (XL16)
-  int res_lo;            // Connect-Four kernel, EPI_CONV2: 1 = the residual has a low-order part (blocks >= 1), 0 = fp16 only (block 0)
-  float* out32;          // EPI_CONV2 (stream), EPI_DENSE (hidden)
-  __half* out16a;        // CONV1: T, CONV2: X16, HEAD: policy features
-  __half* out16b;        // HEAD: value features
+  int res_lo;            // per-layer Connect-Four kernel, EPI_CONV2: 1 = the residual has a low-order part (blocks >= 1), 0 = fp16 only (block 0)
+  float* out32;          // EPI_CONV2 and the stem of the padded layout: fp32 residual stream
+  __half* out16a;        // CONV1: T, CONV2: X16, head conv: policy features
+  __half* out16b;        // head conv: value features
 };
 
+// (`ga` is __grid_constant__: the producer indexes ga.g.off[] with a run-time tap, which is then read from the parameter
+// space in place instead of from a local-memory copy of the whole struct)
 template <int BN, int EPI>
 __global__ void __launch_bounds__(tc::NUM_THREADS, 1)
-az_k_gemm_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW, GemmArgs ga) {
+az_k_gemm_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW, const __grid_constant__ GemmArgs ga) {
   using namespace tc;
   using SmemT = Smem<BN>;
   constexpr int B_BYTES = BN * BK * 2;
@@ -226,8 +231,7 @@ az_k_gemm_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
           mbar_wait(&s.empty[stage], phase ^ 1);
           if (elect_one()) {
             mbar_expect_tx(&s.full[stage], A_BYTES + B_BYTES);
-            if (ga.gemm_k) tma_load_2d(s.a[stage], &tmA, &s.full[stage], kb * BK, tile * BM);
-            else tma_load_2d(s.a[stage], &tmA, &s.full[stage], (kb & 1) * BK, tile * BM + ga.g.off[kb >> 1]);
+            tma_load_2d(s.a[stage], &tmA, &s.full[stage], (kb & 1) * BK, tile * BM + ga.g.off[kb >> 1]);
             tma_load_2d(s.b[stage], &tmW, &s.full[stage], kb * BK, 0);
           }
           __syncwarp();
@@ -272,12 +276,8 @@ az_k_gemm_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
       mbar_wait(&s.tfull[acc], aphase);
       tcgen05_fence_after();
       const int p = tile * BM + quarter * 32 + lane;
-      bool valid;
-      if (EPI == EPI_DENSE) valid = p < rows_used;
-      else {
-        const int r = p % ga.g.board_rows;
-        valid = (p < rows_used) && (r < ga.g.valid_rows) && ((r % ga.g.row_stride) != ga.g.wcols);
-      }
+      const int r = p % ga.g.board_rows;
+      const bool valid = (p < rows_used) && (r < ga.g.valid_rows) && ((r % ga.g.row_stride) != ga.g.wcols);
       const bool in_alloc = p < ga.alloc_rows;
 #pragma unroll 1
       for (int c = 0; c < BN / 32; c++) {
@@ -296,29 +296,21 @@ az_k_gemm_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
             }
           }
         }
-        const bool relu = !(EPI == EPI_DENSE && ga.no_relu);
 #pragma unroll
-        for (int j = 0; j < 32; j++) x[j] = valid ? (relu ? fmaxf(x[j], 0.0f) : x[j]) : 0.0f;
+        for (int j = 0; j < 32; j++) x[j] = valid ? fmaxf(x[j], 0.0f) : 0.0f;
         if (!in_alloc) continue;
-        if (EPI == EPI_CONV2 || EPI == EPI_DENSE || (EPI == EPI_CONV1 && ga.out32 != nullptr)) {
-          if (EPI != EPI_DENSE || valid) {
-            float4* op = reinterpret_cast<float4*>(ga.out32 + (size_t)p * F + c * 32);
+        if (EPI == EPI_CONV2) {
+          float4* op = reinterpret_cast<float4*>(ga.out32 + (size_t)p * F + c * 32);
 #pragma unroll
-            for (int j = 0; j < 8; j++) op[j] = make_float4(x[4 * j], x[4 * j + 1], x[4 * j + 2], x[4 * j + 3]);
-          }
+          for (int j = 0; j < 8; j++) op[j] = make_float4(x[4 * j], x[4 * j + 1], x[4 * j + 2], x[4 * j + 3]);
         }
-        if (EPI != EPI_DENSE) {
-          uint4 o[4];
-          __half2* oh = reinterpret_cast<__half2*>(o);
+        uint4 o[4];
+        __half2* oh = reinterpret_cast<__half2*>(o);
 #pragma unroll
-          for (int j = 0; j < 16; j++) oh[j] = __floats2half2_rn(x[2 * j], x[2 * j + 1]);
-          __half* dst;
-          if (EPI == EPI_HEAD) dst = (c == 0 ? ga.out16a : ga.out16b) + (size_t)p * 32;
-          else dst = ga.out16a + (size_t)p * F + c * 32;
-          uint4* op = reinterpret_cast<uint4*>(dst);
+        for (int j = 0; j < 16; j++) oh[j] = __floats2half2_rn(x[2 * j], x[2 * j + 1]);
+        uint4* op = reinterpret_cast<uint4*>(ga.out16a + (size_t)p * F + c * 32);
 #pragma unroll
-          for (int j = 0; j < 4; j++) op[j] = o[j];
-        }
+        for (int j = 0; j < 4; j++) op[j] = o[j];
       }
       tcgen05_fence_before();
       __syncwarp();
@@ -334,29 +326,20 @@ az_k_gemm_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
 }
 
 // ------------------------------------------------------------------------------------------------
-// Connect-Four tower kernel (row stride W+1 = 8), shared constants.  Each CTA owns HALF of the output channels (64)
-// and keeps that half of the layer's weights resident in shared memory (18 chunks of 64co x 64k, 144 KB); every A
-// stage is reused by three taps: for each kx the producer loads ONE 144-row copy of the activations shifted by
-// dx = 1-kx; because the row stride is 8, the three dy taps are the same copy at row offsets 16 / 8 / 0 = multiples of
-// the 1024-byte swizzle atom, i.e. just a different descriptor start address.  TMA traffic per 128-row tile:
-// 6 stages x 18 KB = 108 KB (5.3x less than the generic kernel).
-// ------------------------------------------------------------------------------------------------
-namespace tc2 {
-constexpr int BM = 128, BNH = 64, BK = 64, AROWS = 144, F = 128;
-constexpr int A_STAGE = AROWS * 128, B_CHUNK = BNH * 128, NCHUNK = 18;
-constexpr int NUM_THREADS = 192;
-}  // namespace tc2
-
-// ------------------------------------------------------------------------------------------------
-// Connect-Four tower kernel, 2-SM version (cta_group::2).  Stall sampling of the 1-SM kernels (profiles/r01_*)
-// shows the tensor pipe starved by SHARED-MEMORY bandwidth, not by L2: an SS-mode M=128,N=128,K=16 MMA reads 8 KB
-// of operands per 64 math cycles, which is all of the 128 B/clk smem port, and the TMA fills share that port.
-// Pairing two CTAs (M = 256 rows per pair) lets each CTA feed its own 128 A rows plus only HALF of B (its resident
-// 64 output channels): 6 KB of operand reads + 1.5 KB of TMA fill per 64 math cycles.
+// Connect-Four tower kernels: 2-CTA clusters (cta_group::2).  A single CTA issuing SS-mode M=128,N=128,K=16 MMAs is
+// starved by SHARED-MEMORY bandwidth, not by L2 (stall sampling, profiles/r01_*): each MMA reads 8 KB of operands per
+// 64 math cycles, which is all of the 128 B/clk smem port, and the TMA fills share that port.  Pairing two CTAs
+// (M = 256 rows per pair) lets each CTA feed its own 128 A rows plus only HALF of B: each CTA owns half of the output
+// channels (64) and keeps that half of the layer's weights resident in shared memory (18 chunks of 64co x 64k, 144 KB).
 // Barrier protocol: TMA loads of both CTAs complete on the LEADER's `full` barrier; the leader's single MMA thread
 // issues tcgen05.mma.cta_group::2 and multicasts tcgen05.commit to both CTAs' `empty` / `tfull` barriers; the 8
 // epilogue warps of the pair arrive on the leader's `tempty`.
 // ------------------------------------------------------------------------------------------------
+namespace tc2 {
+constexpr int BM = 128, BNH = 64, BK = 64;
+constexpr int B_CHUNK = BNH * 128, NCHUNK = 18;
+}  // namespace tc2
+
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
@@ -370,9 +353,6 @@ __device__ __forceinline__ void cluster_sync_all() {
 __device__ __forceinline__ void tma_load_2d_2sm(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1) {
   asm volatile("cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
                ::"r"(smem_u32(dst)), "l"(map), "r"(smem_u32(bar) & 0xFEFFFFFFu), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void tma_prefetch_2d(const CUtensorMap* map, int c0, int c1) {  // warm L2 only, no smem
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global [%0, {%1, %2}];" ::"l"(map), "r"(c0), "r"(c1) : "memory");
 }
 __device__ __forceinline__ void umma_f16_2sm(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
   asm volatile(
@@ -395,285 +375,14 @@ __device__ __forceinline__ void mbar_arrive_cluster(uint64_t* bar, uint32_t cta)
       "}" ::"r"(smem_u32(bar)), "r"(cta) : "memory");
 }
 
-namespace tc3 {
-constexpr int ASTAGES = 3;
-constexpr int NUM_THREADS = 320;  // producer warp, MMA warp, 8 epilogue warps (two per TMEM lane quarter)
-constexpr int EPI_BYTES = 8 * 3072;  // conv2: 8 warps x 3 x 1 KB fp16 out tiles (ring shared by the hi and lo streams);
-                                     // conv1: 8 warps x 2 x 1 KB fp16 out tiles
-constexpr int RES_BYTES = tc2::BM * 128;  // one residual A stage: 128 rows x 64 channels fp16
-struct Smem {
-  uint8_t b[tc2::NCHUNK][tc2::B_CHUNK];
-  uint8_t a[ASTAGES][tc2::A_STAGE];
-  uint8_t ident[1024];  // conv2: this CTA's 8 x 16 slice of the 16 x 16 identity (B operand of the residual MMAs)
-  uint8_t epi[EPI_BYTES];
-  uint64_t full[ASTAGES], empty[ASTAGES], tfull[2], tempty[2], bfull;
-  uint32_t tmem_base;
-  float bias[128];
-};
-}  // namespace tc3
-
-template <int EPI>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(tc3::NUM_THREADS, 1)
-az_k_conv_c4_2sm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW,
-                 const __grid_constant__ CUtensorMap tmO16, const __grid_constant__ CUtensorMap tmOlo,
-                 const __grid_constant__ CUtensorMap tmRhi, const __grid_constant__ CUtensorMap tmRlo, GemmArgs ga) {
-  using namespace tc2;
-  constexpr int BN = 128;
-  constexpr int ASTAGES = tc3::ASTAGES;
-  // every byte of the 227 KB is used, so there is no slack for manual alignment: the dynamic shared memory window starts
-  // 1024-byte aligned (it follows the 1 KB the system reserves per block); trap loudly if that ever stops being true
-  extern __shared__ __align__(1024) uint8_t smem_c4[];
-  if ((smem_u32(smem_c4) & 1023u) != 0u) __trap();
-  tc3::Smem& s = *reinterpret_cast<tc3::Smem*>(smem_c4);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const bool leader = rank == 0;
-  const int rows_used = (*ga.n_boards) * ga.rows_per_board;
-  const int num_ptiles = (rows_used + 2 * BM - 1) / (2 * BM);
-  const int pt0 = blockIdx.x >> 1, pt_step = gridDim.x >> 1;
-
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < ASTAGES; i++) { mbar_init(&s.full[i], 1); mbar_init(&s.empty[i], 1); }
-    for (int i = 0; i < 2; i++) { mbar_init(&s.tfull[i], 1); mbar_init(&s.tempty[i], 16); }
-    mbar_init(&s.bfull, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  float* bias_s = s.bias;
-  if (threadIdx.x >= 64 && threadIdx.x < 64 + BN) bias_s[threadIdx.x - 64] = ga.bias[threadIdx.x - 64];
-  if (EPI == tc::EPI_CONV2 && threadIdx.x >= 192 && threadIdx.x < 192 + 64) {
-    // identity slice: the residual MMAs are M = 256, N = 16, K = 16 with D columns [c, c+16) += A[:, c..c+15] . I16; this
-    // CTA supplies output columns rank*8 .. rank*8+7, i.e. B[n'][k] = (k == rank*8 + n'), un-swizzled K-major core matrices
-    const int i = threadIdx.x - 192;  // 64 x 4 bytes = the 256-byte slice
-    const int n = (i & 31) >> 2, khalf = i >> 5, kk = (i & 3) * 2;  // 16 B per row: 4 words of 2 halves
-    const int k0 = khalf * 8 + kk, kone = (int)rank * 8 + n;
-    const uint32_t w = (k0 == kone ? 0x3C00u : 0u) | (k0 + 1 == kone ? 0x3C000000u : 0u);
-    *reinterpret_cast<uint32_t*>(s.ident + khalf * 128 + n * 16 + (i & 3) * 4) = w;
-    fence_proxy_async();
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&s.tmem_base)), "r"(256u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  tcgen05_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  tcgen05_fence_after();
-  const uint32_t tmem_base = s.tmem_base;
-  // Programmatic dependent launch: let the next layer's CTAs be scheduled as SMs drain; everything above and the
-  // weight load below do not depend on the previous layer, activations are only touched after griddepcontrol.wait.
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-
-  if (warp == 0) {
-    if (pt0 < num_ptiles) {  // ===== TMA producer (both CTAs; warp-uniform, one elected lane issues) =====
-      if (elect_one()) {
-        if (leader) mbar_expect_tx(&s.bfull, 2 * NCHUNK * B_CHUNK);
-        for (int ch = 0; ch < NCHUNK; ch++) tma_load_2d_2sm(s.b[ch], &tmW, &s.bfull, ch * BK, (int)rank * BNH);
-      }
-      __syncwarp();
-      asm volatile("griddepcontrol.wait;" ::: "memory");
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int pt = pt0; pt < num_ptiles; pt += pt_step) {
-        const int row0 = pt * 2 * BM + (int)rank * BM;
-        // conv2 interleaves its residual stages (this CTA's 128 rows of the block input, 64 channels at a time, hi then lo
-        // part) with the first conv stages: C0 R0 C1 R1 C2 [R2 C3 R3] C.. -- a residual stage is consumed ~6x faster than
-        // a conv stage, and four in a row would leave the 3-slot ring only ~0.2 us of prefetch distance
-        const int nres = (EPI == tc::EPI_CONV2) ? (ga.res_lo ? 4 : 2) : 0;
-        for (int q = 0; q < 6 + nres; q++) {
-          const bool isres = q < 2 * nres && (q & 1);
-          const int st = q < 2 * nres ? (q >> 1) : q - nres;  // residual stage index or conv stage index
-          mbar_wait(&s.empty[stage], phase ^ 1);
-          if (elect_one()) {
-            if (isres) {
-              if (leader) mbar_expect_tx(&s.full[stage], 2 * tc3::RES_BYTES);
-              tma_load_2d_2sm(s.a[stage], (st >> 1) ? &tmRlo : &tmRhi, &s.full[stage], (st & 1) * BK, row0);
-            } else {
-              if (leader) mbar_expect_tx(&s.full[stage], 2 * A_STAGE);
-              tma_load_2d_2sm(s.a[stage], &tmA, &s.full[stage], (st & 1) * BK, row0 - 8 + (1 - (st >> 1)));
-            }
-          }
-          __syncwarp();
-          if (++stage == ASTAGES) { stage = 0; phase ^= 1; }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    if (leader && pt0 < num_ptiles) {  // ===== MMA issuer (leader CTA only; warp-uniform, one elected lane issues) =====
-      constexpr uint32_t IDESC = (1u << 4) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)((2 * BM) >> 4) << 24);  // M = 256, N = 128
-      mbar_wait(&s.bfull, 0);
-      tcgen05_fence_after();
-      int stage = 0;
-      uint32_t phase = 0;
-      int it = 0;
-      for (int pt = pt0; pt < num_ptiles; pt += pt_step, it++) {
-        const int acc = it & 1;
-        const uint32_t aphase = (it >> 1) & 1;
-        mbar_wait(&s.tempty[acc], aphase ^ 1);
-        tcgen05_fence_after();
-        const uint32_t tmem_d = tmem_base + acc * BN;
-        // skip connection on the tensor core (conv2): x = hi (+ lo) is added to the accumulator by 16-column identity MMAs
-        // (resnet.jl:55-62: relu(x + conv2(...))), so the epilogue never reads the residual
-        constexpr uint32_t IDESC_R = (1u << 4) | ((uint32_t)(16 >> 3) << 17) | ((uint32_t)((2 * BM) >> 4) << 24);  // M = 256, N = 16
-        const uint64_t idsc = umma_desc_interleave(smem_u32(s.ident), 128u, 256u);
-        const int nres = (EPI == tc::EPI_CONV2) ? (ga.res_lo ? 4 : 2) : 0;
-        for (int q = 0; q < 6 + nres; q++) {
-          const bool isres = q < 2 * nres && (q & 1);
-          const int st = q < 2 * nres ? (q >> 1) : q - nres;
-          const int kx = st >> 1, half = st & 1;
-          mbar_wait(&s.full[stage], phase);
-          tcgen05_fence_after();
-          const uint32_t abase = smem_u32(s.a[stage]);
-          if (elect_one()) {
-            if (isres) {
-              const uint64_t adesc = umma_desc_sw128(abase);
-#pragma unroll
-              for (int k = 0; k < BK / 16; k++)
-                umma_f16_2sm(tmem_d + (uint32_t)(half * BK + k * 16), adesc + (uint64_t)(k * 2), idsc, IDESC_R, 1u);
-            } else {
-#pragma unroll
-              for (int ky = 0; ky < 3; ky++) {
-                const uint64_t adesc = umma_desc_sw128(abase + (uint32_t)(8 + 8 * (1 - ky)) * 128u);
-                const uint64_t bdesc = umma_desc_sw128(smem_u32(s.b[(ky * 3 + kx) * 2 + half]));
-#pragma unroll
-                for (int k = 0; k < BK / 16; k++)
-                  umma_f16_2sm(tmem_d, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), IDESC, (st | ky | k) ? 1u : 0u);
-              }
-            }
-            umma_commit_2sm(&s.empty[stage]);
-            if (q == 5 + nres) umma_commit_2sm(&s.tfull[acc]);
-          }
-          __syncwarp();
-          if (++stage == ASTAGES) { stage = 0; phase ^= 1; }
-        }
-      }
-    }
-  } else {  // ===== epilogue warps 2..9 (both CTAs): own 128 rows x 128 channels =====
-    // TMEM gives each thread one ROW.  Writing rows straight to global memory costs 32 distinct 128-B lines per warp
-    // instruction (the LSU tag pipeline became the bottleneck), so each 32x16 block goes through a per-warp swizzled smem
-    // tile and leaves by a TMA bulk-tensor store.  Two warps share a TMEM lane quarter (64 columns each).
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    const int quarter = warp & 3;
-    const int colhalf = (warp - 2) >> 2;
-    if (EPI == tc::EPI_CONV1) {
-      // conv1 epilogue: every thread owns one output ROW (TMEM lane).  bias + ReLU + pad-row zeroing + fp16 conversion
-      // happen in registers, the 32 x 16 fp16 block goes to a 1 KB SWIZZLE_32B smem tile (2 conflict-free 16-byte
-      // stores per thread) and leaves through ONE TMA bulk-tensor store: no smem transpose and no per-row STGs in the
-      // L1TEX data pipe that the tensor core's operand reads share.  Two tiles per warp, alternating.
-      uint8_t* tile0 = s.epi + (warp - 2) * 2048;  // 2 x 1024 B per warp
-      int it = 0;
-      for (int pt = pt0; pt < num_ptiles; pt += pt_step, it++) {
-        const int acc = it & 1;
-        const uint32_t aphase = (it >> 1) & 1;
-        const int prow0 = pt * 2 * BM + (int)rank * BM + quarter * 32;
-        const int p = prow0 + lane;
-        const int r = p % ga.g.board_rows;
-        const bool valid = (p < rows_used) && (r < ga.g.valid_rows) && ((r % ga.g.row_stride) != ga.g.wcols);
-        mbar_wait(&s.tfull[acc], aphase);
-        tcgen05_fence_after();
-#pragma unroll
-        for (int sc = 0; sc < 4; sc++) {
-          const int col = colhalf * 64 + sc * 16;
-          uint32_t v[16];
-          tmem_ld16(tmem_base + acc * BN + col + ((uint32_t)(quarter * 32) << 16), v);
-          uint4 o[2];
-          __half2* oh = reinterpret_cast<__half2*>(o);
-#pragma unroll
-          for (int j = 0; j < 8; j++) {
-            float x0 = __uint_as_float(v[2 * j]) + bias_s[col + 2 * j];
-            float x1 = __uint_as_float(v[2 * j + 1]) + bias_s[col + 2 * j + 1];
-            x0 = valid ? fmaxf(x0, 0.f) : 0.f;
-            x1 = valid ? fmaxf(x1, 0.f) : 0.f;
-            oh[j] = __floats2half2_rn(x0, x1);
-          }
-          uint8_t* tile = tile0 + (sc & 1) * 1024;
-          if (lane == 0) tma_store_wait_read<1>();  // the store issued two blocks ago has finished reading this tile
-          __syncwarp();
-          const int sw = (lane >> 2) & 1;  // SWIZZLE_32B: 16-byte chunk index ^= bit 7 of the byte address (row >> 2)
-          *reinterpret_cast<uint4*>(tile + lane * 32 + ((0 ^ sw) << 4)) = o[0];
-          *reinterpret_cast<uint4*>(tile + lane * 32 + ((1 ^ sw) << 4)) = o[1];
-          fence_proxy_async();
-          __syncwarp();
-          if (lane == 0 && !(ga.debug & 4)) { tma_store_2d(&tmO16, tile, col, prow0); tma_store_commit(); }
-        }
-        tcgen05_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(&s.tempty[acc], 0);
-      }
-      if (lane == 0) tma_store_wait_all();
-      __syncwarp();
-    } else {
-      // conv2 epilogue: the accumulator already holds x + conv2 (identity MMAs above), so this is the conv1 epilogue plus
-      // the split of the fp32 result y = relu(acc + bias) into hi = fp16(y) (the next conv's input) and lo = fp16(y - hi)
-      // (the rest of the skip path's precision: hi + lo carries ~22 mantissa bits).  Both leave through TMA stores from a
-      // ring of three 1 KB SWIZZLE_32B tiles per warp, one bulk group per store.
-      uint8_t* tiles = s.epi + (warp - 2) * 3072;
-      int ring = 0;
-      const int sw = (lane >> 2) & 1;  // SWIZZLE_32B: 16-byte chunk index ^= bit 7 of the byte address (row >> 2)
-      int it = 0;
-      for (int pt = pt0; pt < num_ptiles; pt += pt_step, it++) {
-        const int acc = it & 1;
-        const uint32_t aphase = (it >> 1) & 1;
-        const int prow0 = pt * 2 * BM + (int)rank * BM + quarter * 32;
-        const int p = prow0 + lane;
-        const int r = p % ga.g.board_rows;
-        const bool valid = (p < rows_used) && (r < ga.g.valid_rows) && ((r % ga.g.row_stride) != ga.g.wcols);
-        mbar_wait(&s.tfull[acc], aphase);
-        tcgen05_fence_after();
-#pragma unroll
-        for (int sc = 0; sc < 4; sc++) {
-          const int col = colhalf * 64 + sc * 16;
-          uint32_t v[16];
-          tmem_ld16(tmem_base + acc * BN + col + ((uint32_t)(quarter * 32) << 16), v);
-          uint4 oh4[2], ol4[2];
-          __half2* oh = reinterpret_cast<__half2*>(oh4);
-          __half2* ol = reinterpret_cast<__half2*>(ol4);
-#pragma unroll
-          for (int j = 0; j < 8; j++) {
-            float x0 = __uint_as_float(v[2 * j]) + bias_s[col + 2 * j];
-            float x1 = __uint_as_float(v[2 * j + 1]) + bias_s[col + 2 * j + 1];
-            x0 = valid ? fmaxf(x0, 0.f) : 0.f;
-            x1 = valid ? fmaxf(x1, 0.f) : 0.f;
-            const __half2 h = __floats2half2_rn(x0, x1);
-            const float2 hf = __half22float2(h);
-            oh[j] = h;
-            ol[j] = __floats2half2_rn(x0 - hf.x, x1 - hf.y);
-          }
-#pragma unroll
-          for (int part = 0; part < 2; part++) {
-            uint8_t* tile = tiles + ring * 1024;
-            if (++ring == 3) ring = 0;
-            if (lane == 0) tma_store_wait_read<2>();  // the store issued three stores ago has finished reading this tile
-            __syncwarp();
-            const uint4* o = part ? ol4 : oh4;
-            *reinterpret_cast<uint4*>(tile + lane * 32 + ((0 ^ sw) << 4)) = o[0];
-            *reinterpret_cast<uint4*>(tile + lane * 32 + ((1 ^ sw) << 4)) = o[1];
-            fence_proxy_async();
-            __syncwarp();
-            if (lane == 0) { tma_store_2d(part ? &tmOlo : &tmO16, tile, col, prow0); tma_store_commit(); }
-          }
-        }
-        tcgen05_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(&s.tempty[acc], 0);
-      }
-      if (lane == 0) tma_store_wait_all();
-      __syncwarp();
-    }  // EPI_CONV2
-  }
-  tcgen05_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  if (warp == 1) {
-    tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(256u) : "memory");
-  }
-}
-
 // ------------------------------------------------------------------------------------------------
-// Connect-Four tower kernel, "y-row" version (round 2).  What the round-1 kernel above leaves on the table
-// (profiles/r01_final2_*): 56 MMA rows per 42 valid cells (25 % of the issued MMAs are padding), tile-round
-// quantisation (604 tiles over 74 CTA pairs = 8.2 -> 9 rounds), three shifted shared-memory copies of every activation
-// row, and zeroing / storing of pad rows.
+// Connect-Four tower conv, one layer per launch ("y-row" kernel, round 2; AZ_TOWER=layer).  The persistent kernel below
+// runs the same MMAs in the same order for every output row, so with the same residual format (AZ_LO=16) its outputs must
+// equal this kernel's bit for bit: this kernel is the reference test_persistent_tower_equals_per_layer_kernels checks
+// the persistent one against.
+// Why not the padded layout on Connect Four (round 1, profiles/r01_final2_*): 56 MMA rows per 42 valid cells (25 % of
+// the issued MMAs are padding), tile-round quantisation (604 tiles over 74 CTA pairs = 8.2 -> 9 rounds), three shifted
+// shared-memory copies of every activation row, and zeroing / storing of pad rows.
 //
 // Here the activations are stored DENSE in HBM -- row(b, y, x) = b*42 + y*7 + x, 128 fp16 channels -- and seen by TMA
 // as a 4-D tensor (channel, x, y, board).  One A stage = one board ROW y of 16 consecutive boards, 64 channels:
@@ -700,8 +409,8 @@ az_k_conv_c4_2sm(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 //     board, so the epilogue needs no validity masking; x-slot 7 and boards past the allocation are clipped by the TMA
 //     store (out-of-bounds elements of a store box are not written).
 // Weights (this CTA's 64 output channels, 144 KB) stay resident in shared memory; the skip connection of conv2 is
-// added on the tensor core by identity MMAs over the fp16 hi + lo residual stream as in the round-1 kernel (its A
-// stages are loaded with the same x = -1 origin and read one row in).
+// added on the tensor core by identity MMAs over the fp16 hi + lo residual stream, so the epilogue never reads the
+// residual (its A stages are loaded with the same x = -1 origin and read one row in).
 // ------------------------------------------------------------------------------------------------
 namespace yr {
 constexpr int NBOARD = 16;            // boards per CTA tile
@@ -947,7 +656,7 @@ az_k_conv_yrow(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           *reinterpret_cast<uint4*>(tile + lane * 32 + ((1 ^ sw) << 4)) = o[1];
           fence_proxy_async();
           __syncwarp();
-          if (lane == 0 && !(ga.debug & 4)) { tma_store_4d(part ? &tmOlo : &tmO16, tile, col, 0, j, bq); tma_store_commit(); }
+          if (lane == 0) { tma_store_4d(part ? &tmOlo : &tmO16, tile, col, 0, j, bq); tma_store_commit(); }
         }
       }
       tcgen05_fence_before();
@@ -1008,10 +717,10 @@ struct Smem {
 // first segments of the next layer need has been in memory for about half a layer, the producer has already put the next
 // layer's first A stages into the ring, and the only wait left at the boundary is the first weight chunk.
 struct Seg { int g, j_lo, j_hi; };
-__device__ __forceinline__ Seg segment(int k, int nseg, int u0, int u1, bool natural) {
+__device__ __forceinline__ Seg segment(int k, int nseg, int u0, int u1) {
   int i = k;
-  if (!natural && nseg >= 2 && u1 % 6 != 0) i = (k == 0) ? nseg - 1 : k - 1;   // (a range that ends on a group boundary has no
-                                                                              // reader above: its first segment goes first)
+  if (nseg >= 2 && u1 % 6 != 0) i = (k == 0) ? nseg - 1 : k - 1;   // (a range that ends on a group boundary has no
+                                                                  // reader above: its first segment goes first)
   Seg sg;
   sg.g = u0 / 6 + i;
   sg.j_lo = (i == 0) ? u0 - sg.g * 6 : 0;
@@ -1082,7 +791,6 @@ az_k_tower_yrow(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
   const uint32_t rank = cluster_ctarank();
   const bool leader = rank == 0;
   const int pair = blockIdx.x >> 1, npairs = gridDim.x >> 1;
-  const bool use_lo = !(ga.debug & 8);   // AZ_TOWER_DEBUG=8 (timing experiments only): fp16-only skip stream, no low-order part
   const bool lo8 = ga.lo8 != 0;          // low-order part of the skip stream as e4m3 bytes (default) or fp16 (AZ_LO=16)
 
   if (threadIdx.x == 0) {
@@ -1142,7 +850,6 @@ az_k_tower_yrow(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
   }
   const int Up = u1 - u0;                                         // units per layer
   const int nseg = has_work ? (u1 - 1) / H - u0 / H + 1 : 0;
-  const bool natural = (ga.debug & 16) != 0;                      // AZ_TOWER_DEBUG=16 (A/B runs): segments in range order
   unsigned long long* const done_up = done + 128;                 // row u1-1 of a layer stored (read by the pair above); `done`: row u0
   cluster_sync_all();  // `base` is read by both CTAs before any warp of the pair can add to the counter
 
@@ -1164,7 +871,7 @@ az_k_tower_yrow(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
       const CUtensorMap* mA = conv2 ? &tmT : &tmX;
       int cum = 0;   // units of this layer's segments up to and including the current one (processing order)
       for (int k = 0; k < nseg; k++) {
-        const tw::Seg sg = tw::segment(k, nseg, u0, u1, natural);
+        const tw::Seg sg = tw::segment(k, nseg, u0, u1);
         const int g = sg.g, j_lo = sg.j_lo, j_hi = sg.j_hi;
         cum += j_hi - j_lo;
         const bool lo_halo = q_lo >= 0 && g * H + j_lo == u0;   // bottom halo row: produced by the pair below in layer l-1
@@ -1194,7 +901,7 @@ az_k_tower_yrow(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
             fence_proxy_async();
             hi_ok = true;
           }
-          const int nres = (conv2 && y >= j_lo && y < j_hi) ? ((l > 1 && use_lo) ? (lo8 ? 3 : 4) : 2) : 0;
+          const int nres = (conv2 && y >= j_lo && y < j_hi) ? (l > 1 ? (lo8 ? 3 : 4) : 2) : 0;
           for (int q = 0; q < 2 + nres; q++) {
             int kind, half;
             tw::stage_of(q, nres, lo8, kind, half);
@@ -1249,7 +956,7 @@ az_k_tower_yrow(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
         const bool conv2 = (l & 1) != 0;
         uint32_t wready = 0;   // bit ch: this layer's weight chunk ch has been waited for
         for (int k = 0; k < nseg; k++) {
-          const tw::Seg sg = tw::segment(k, nseg, u0, u1, natural);
+          const tw::Seg sg = tw::segment(k, nseg, u0, u1);
           const int j_lo = sg.j_lo, j_hi = sg.j_hi;
           const int y_lo = max(0, j_lo - 1), y_hi = min(H - 1, j_hi);
           for (int y = y_lo; y <= y_hi; y++) {
@@ -1259,7 +966,7 @@ az_k_tower_yrow(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
               mbar_wait(&s.tempty[n & 3], ((uint32_t)(n >> 2) & 1u) ^ 1u);
             }
             tcgen05_fence_after();
-            const int nres = (conv2 && y >= j_lo && y < j_hi) ? ((l > 1 && use_lo) ? (lo8 ? 3 : 4) : 2) : 0;
+            const int nres = (conv2 && y >= j_lo && y < j_hi) ? (l > 1 ? (lo8 ? 3 : 4) : 2) : 0;
             for (int q = 0; q < 2 + nres; q++) {
               int kind, half;
               tw::stage_of(q, nres, lo8, kind, half);
@@ -1340,11 +1047,11 @@ az_k_tower_yrow(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
     int n = 0;
     for (int l = 0; l < num_layers; l++) {
       const bool conv2 = (l & 1) != 0;
-      const bool want_lo = conv2 && l != num_layers - 1 && use_lo;   // nobody reads the low-order part of the last block's output
+      const bool want_lo = conv2 && l != num_layers - 1;   // nobody reads the low-order part of the last block's output
       const float* __restrict__ bias_g = ga.bias + (size_t)l * 128 + colhalf * 64;
       const CUtensorMap* mO = conv2 ? &tmXo : &tmTo;
       for (int k = 0; k < nseg; k++) {
-        const tw::Seg sg = tw::segment(k, nseg, u0, u1, natural);
+        const tw::Seg sg = tw::segment(k, nseg, u0, u1);
         const int g = sg.g;
         for (int j = sg.j_lo; j < sg.j_hi; j++, n++) {
           const int bq = g * 2 * NB + (int)rank * NB + quarter * 4;
@@ -1387,7 +1094,7 @@ az_k_tower_yrow(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
               for (int c = 0; c < 4; c++) *reinterpret_cast<uint4*>(tile + lane * 64 + ((c ^ sw) << 4)) = o[c];
               fence_proxy_async();
               __syncwarp();
-              if (lane == 0 && !(ga.debug & 4)) { tma_store_4d(part ? &tmXLo : mO, tile, col, 0, j, bq); tma_store_commit(); }
+              if (lane == 0) { tma_store_4d(part ? &tmXLo : mO, tile, col, 0, j, bq); tma_store_commit(); }
             }
           }
           if (want_lo && lo8) {  // one 32-row x 64-byte tile of e4m3 bytes (channels colhalf*64 .. +63)
@@ -1397,7 +1104,7 @@ az_k_tower_yrow(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
             for (int c = 0; c < 4; c++) *reinterpret_cast<uint4*>(tile + lane * 64 + ((c ^ sw) << 4)) = l8[c];
             fence_proxy_async();
             __syncwarp();
-            if (lane == 0 && !(ga.debug & 4)) { tma_store_4d(&tmXL8o, tile, colhalf * 64, 0, j, bq); tma_store_commit(); }
+            if (lane == 0) { tma_store_4d(&tmXL8o, tile, colhalf * 64, 0, j, bq); tma_store_commit(); }
           }
           tcgen05_fence_before();
           __syncwarp();
@@ -1426,99 +1133,9 @@ az_k_tower_yrow(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
 }
 
 // ------------------------------------------------------------------------------------------------
-// stem: leaf states -> im2col rows -> tcgen05 GEMM.  The first conv (3x3, C_in -> 128, folded BN, ReLU) has K = 9*C_in
-// (27 for Connect Four): az_k_im2col writes, for every padded board row, the 9*C_in input-plane values of its 3x3
-// neighbourhood as one 128-byte fp16 row (K padded to 64), straight from the game's vectorize_state (no host round
-// trip; replaces GI.vectorize_state + Flux.batch + convert_input, src/networks/network.jl:310-312); the conv itself is
-// then one az_k_gemm_tc<128, EPI_CONV1> launch with a single K block.  One warp per board.
-// ------------------------------------------------------------------------------------------------
-template <class G>
-__global__ void __launch_bounds__(128) az_k_im2col(const AzEnv* __restrict__ envs, const int32_t* __restrict__ n_boards,
-                                                   __half* __restrict__ out /* [rows][64] */, int dense) {
-  constexpr int W = G::XW, H = G::XH, C = G::XC, NX = W * H * C;
-  const int RS = dense ? W : W + 1, BS = dense ? W * H : (W + 1) * (H + 1);  // dense rows (y-row tower) or padded NHWC
-  __shared__ float xs[4][NX];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int b = blockIdx.x * 4 + warp;
-  if (b >= *n_boards) return;
-  float* x = xs[warp];
-  if (lane == 0) G::vectorize(envs[b], x);
-  __syncwarp();
-  uint4* ob = reinterpret_cast<uint4*>(out + (size_t)b * BS * 64);
-  for (int i = lane; i < BS * 8; i += 32) {  // 8 x 16-byte chunks per row
-    const int r = i >> 3, q = i & 7, yy = r / RS, xx = r % RS;
-    __align__(16) __half h[8];
-#pragma unroll
-    for (int j = 0; j < 8; j++) {
-      const int k = q * 8 + j;  // k = tap*C + c, tap = ky*3 + kx
-      float v = 0.0f;
-      if (k < 9 * C && yy < H && xx < W) {
-        const int tap = k / C, c = k % C, ky = tap / 3, kx = tap % 3;
-        // Flux Conv is a true convolution: tap (kx,ky) reads the input at (x + 1 - kx, y + 1 - ky)
-        const int ix = xx + 1 - kx, iy = yy + 1 - ky;
-        if (ix >= 0 && ix < W && iy >= 0 && iy < H) v = x[ix + W * iy + W * H * c];
-      }
-      h[j] = __float2half_rn(v);
-    }
-    ob[i] = *reinterpret_cast<const uint4*>(h);
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// finalize: policy dense + softmax + legal-action mask + renormalisation (resnet.jl:83-84, network.jl:264-271),
-// value output tanh(w2 . hidden + b2) (resnet.jl:89-90).  One warp per board.
-// ------------------------------------------------------------------------------------------------
-struct FinalArgs {
-  const float* logit;  // [boards][128]: policy logits in columns 0..A-1 (bias already added by the GEMM epilogue)
-  const float* hid;    // value hidden [boards][128]
-  const float* wv2;    // [128]
-  const float* bv2;    // [1]
-  float* logit_out;    // parity hook (az_net_forward_logits): [boards][A] pre-softmax policy logits, or null
-  float* vpre_out;     // parity hook: [boards] pre-tanh value, or null
-};
-// softmax + legal-action mask + renormalisation (resnet.jl:84, network.jl:264-271), value = tanh(w2 . hidden + b2)
-// (resnet.jl:89-90).  8 lanes per board.
-template <class G>
-__global__ void __launch_bounds__(256) az_k_finalize(const AzEnv* __restrict__ envs, const int32_t* __restrict__ n_boards, FinalArgs fa,
-                                                     float* __restrict__ P, float* __restrict__ V, float* __restrict__ Pinv) {
-  constexpr int A = G::A;
-  const int gid = blockIdx.x * blockDim.x + threadIdx.x;
-  const int b = gid >> 3, sub = gid & 7;
-  const bool active = b < *n_boards;
-  float vacc = 0.0f;
-  if (active) {
-    const float4* hp = reinterpret_cast<const float4*>(fa.hid + (size_t)b * 128 + sub * 16);
-    const float4* wp = reinterpret_cast<const float4*>(fa.wv2 + sub * 16);
-#pragma unroll
-    for (int q = 0; q < 4; q++) { const float4 h = hp[q], w = wp[q]; vacc += h.x * w.x + h.y * w.y + h.z * w.z + h.w * w.w; }
-  }
-#pragma unroll
-  for (int off = 4; off >= 1; off >>= 1) vacc += __shfl_xor_sync(0xffffffffu, vacc, off);
-  if (active && sub == 0) {
-    float lg[A], m = -3.0e38f;
-#pragma unroll
-    for (int a = 0; a < A; a++) { lg[a] = fa.logit[(size_t)b * 128 + a]; m = fmaxf(m, lg[a]); }
-    float se = 0.0f;
-#pragma unroll
-    for (int a = 0; a < A; a++) { lg[a] = expf(lg[a] - m); se += lg[a]; }
-    const uint32_t legal = G::legal_mask(envs[b]);
-    float sp = 0.0f;
-#pragma unroll
-    for (int a = 0; a < A; a++) { lg[a] = ((legal >> a) & 1u) ? lg[a] / se : 0.0f; sp += lg[a]; }
-#pragma unroll
-    for (int a = 0; a < A; a++) P[(size_t)b * A + a] = lg[a] / (sp + 1.1920929e-07f);  // eps(Float32), network.jl:268
-    V[b] = tanhf(vacc + fa.bv2[0]);
-    if (Pinv) Pinv[b] = 1.0f - sp;
-    if (fa.vpre_out) fa.vpre_out[b] = vacc + fa.bv2[0];
-    if (fa.logit_out) {
-#pragma unroll
-      for (int a = 0; a < A; a++) fa.logit_out[(size_t)b * A + a] = fa.logit[(size_t)b * 128 + a];
-    }
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// Fused stem (round 2): leaf states -> first conv, ONE kernel.  The im2col rows are never written to HBM: four builder
+// Stem (round 2): leaf states -> first conv (3x3, C_in -> 128, folded BN, ReLU; K = 9*C_in = 27 for Connect Four, padded
+// to one 64-wide K block), ONE kernel, straight from the game's vectorize_state (no host round trip; replaces
+// GI.vectorize_state + Flux.batch + convert_input, src/networks/network.jl:310-312).  The im2col rows are never written to HBM: four builder
 // warps (one thread per tile row) assemble the 128 x 64 fp16 A tile of the first conv directly in shared memory in the
 // SWIZZLE_128B K-major layout the tensor core reads (a row is exactly one 128-byte swizzle row), double buffered
 // against the MMA (4 x tcgen05.mma M=128,N=128,K=16 per tile) and the epilogue of the previous tile.  Saves the 15 MB
@@ -1696,7 +1313,7 @@ az_k_stem(const AzEnv* __restrict__ envs, const __grid_constant__ CUtensorMap tm
 
 // ------------------------------------------------------------------------------------------------
 // Head 1x1 convs (round 2): both heads' Conv1x1(128 -> 32) + BatchNorm + ReLU as one N = 64 GEMM over the tower's output rows.
-// Replaces az_k_gemm_tc<64, EPI_HEAD> for this job: the 16 KB of weights stay resident (loaded once per CTA), the A ring
+// Unlike the generic GEMM kernel, the 16 KB of weights stay resident (loaded once per CTA), the A ring
 // holds four 16 KB stages (two tiles in flight), the fp16 feature rows leave as 2 KB bulk copies (a feature row is 64
 // contiguous bytes, so 32 rows of a head are one contiguous chunk), and at 80 KB of shared memory two CTAs share an SM.
 // ------------------------------------------------------------------------------------------------
@@ -2064,8 +1681,8 @@ template <class G>
 struct ResNetImpl : az_net {
   az_resnet_hp hp{};
   static constexpr int F = 128, W = G::XW, H = G::XH, C = G::XC, A = G::A, WH = W * H;
-  // activation row layout, fixed at init(): padded NHWC (row stride W+1, one zero row per board) for the generic 9-tap
-  // kernel and the round-1 Connect-Four kernel, or DENSE rows (b*W*H + y*W + x) for the y-row tower kernel
+  // activation row layout, fixed at init(): DENSE rows (b*W*H + y*W + x) for the Connect-Four tower kernels
+  // (C4_TOWER && num_blocks > 0), otherwise padded NHWC (row stride W+1, one zero row per board) for the generic 9-tap kernel
   bool dense = false;
   int RS = W + 1;                                              // rows per board row
   int BS = (W + 1) * (H + 1);                                  // rows per board
@@ -2075,32 +1692,23 @@ struct ResNetImpl : az_net {
   // device weights
   __half* d_wstem = nullptr; float* d_bstem = nullptr;   // stem weights Wt[co][64] (k = tap*C + c, zero padded)
   __half* d_wpol = nullptr; float* d_bpol = nullptr;     // policy dense as a GEMM: Wt[64 (A used)][KD]
-  CUtensorMap mapWstem{}, mapWpol{}, mapX0{}, mapHp{};
-  __half* d_x0 = nullptr;       // im2col rows [alloc_rows][64]
-  float* d_logit = nullptr;     // [boards][128]
+  CUtensorMap mapWstem{}, mapWpol{}, mapHp{};
   std::vector<__half*> d_wconv; std::vector<float*> d_bconv;   // per-layer views into d_wall / d_ball
   __half* d_wall = nullptr; float* d_ball = nullptr;            // all tower layers: Wt[l][co][tap*F + ci], bias[l][co]
   unsigned long long* d_done = nullptr;                          // persistent tower: per-pair layer counters (never reset)
   CUtensorMap mapWall{};                                         // [L*128][1152] fp16, 64 x 64 boxes
-  bool persistent = true;      // AZ_TOWER=layer: one launch per conv layer (round-2a kernel) instead of the whole-tower kernel
-  bool coop_launch = true;     // cooperative launch of the persistent kernel (co-residency of all CTA pairs guaranteed)
+  bool persistent = true;      // AZ_TOWER=layer: one launch per conv layer (the reference kernel) instead of the whole-tower kernel
   size_t smem_tower = 0, smem_stem = 0;
-  bool fused = true;           // AZ_FUSED=0: round-1 im2col + GEMM stem and separate dense / finalize launches
   __half *d_wh = nullptr, *d_wd = nullptr;
   float *d_bh = nullptr, *d_bd = nullptr, *d_wv2 = nullptr, *d_bv2 = nullptr;
   std::vector<CUtensorMap> mapW;
   CUtensorMap mapWh{}, mapWd{};
   // activations (allocated for max_rows on first use)
   int act_boards = 0, alloc_rows = 0, alloc_boards = 0;
-  float *d_x32 = nullptr, *d_hid = nullptr;
+  float* d_x32 = nullptr;                 // generic tower: fp32 residual stream
   __half *d_x16 = nullptr, *d_t16 = nullptr, *d_hp = nullptr, *d_hv = nullptr;
   CUtensorMap mapX{}, mapT{}, mapHv{};
-  CUtensorMap mapX2{}, mapT2{};          // Connect-Four tower kernel: 144-row A boxes
-  CUtensorMap mapTo{}, mapXo{};          // TMA-store targets: 32-row x 16-column fp16 boxes, SWIZZLE_32B
-  CUtensorMap mapX32{};                  // (generic tower only) fp32 residual stream
   __half* d_xl16 = nullptr;              // Connect-Four tower: low-order part of the block outputs (x = X16 + XL16)
-  CUtensorMap mapXr{}, mapXLr{};         // residual A stages: 128-row x 64-channel boxes of X16 / XL16
-  CUtensorMap mapXLo{};                  // TMA-store target for XL16
   std::vector<CUtensorMap> mapW2;        // 64co x 64k weight boxes
   // y-row tower: 4-D (channel, x, y, board) views of the dense activations
   CUtensorMap map4X{}, map4T{}, map4XL{};        // loads: box (64 ch, 8 x, 1 y, 16 boards), SWIZZLE_128B, zero fill outside
@@ -2111,14 +1719,10 @@ struct ResNetImpl : az_net {
   CUtensorMap mapXo64{};                           // stem stores: 2-D [rows][128] fp16, box (32 ch, 32 rows), SWIZZLE_64B
   CUtensorMap map4Xo64{}, map4To64{}, map4XLo64{};  // stores of the persistent kernel: box (32 ch, 8 x, 1 y, 4 boards), SWIZZLE_64B
   static constexpr bool C4_TOWER = (W + 1) == 8 && H == 6;
-  size_t smem_2sm = 0, smem_yrow = 0;
+  size_t smem_yrow = 0;
   ConvGeom geom{};
   bool loaded = false;
-  int tower_debug = 0;         // AZ_TOWER_DEBUG=1: every conv uses the conv1 epilogue (timing experiments only)
-  bool use_pdl = true;         // AZ_NO_PDL=1: plain stream-ordered tower launches
-  static constexpr bool two_sm = true;
-  bool generic_tower = false;  // AZ_GENERIC_TOWER=1: use the generic 9-tap kernel for Connect Four too (A/B comparison)
-  size_t smem128 = 0, smem64 = 0;
+  size_t smem128 = 0;
   // profiling: 4 events per evaluation (start, tower begin, tower end, end)
   // The event ring is drained (stream sync + accumulate) whenever it fills, so EVERY evaluation of a profiled pass is
   // counted whatever its length (round 1 truncated at the ring size and overstated the roofline for long passes).
@@ -2156,7 +1760,7 @@ struct ResNetImpl : az_net {
   int get_profile(double* tower_ms, int64_t* tower_launches, double* total_ms, int64_t* evals) override {
     prof_drain();
     if (tower_ms) *tower_ms = prof_tower_ms;
-    if (tower_launches) *tower_launches = prof_drained * ((dense && persistent && hp.num_blocks > 0) ? 1 : 2 * hp.num_blocks);
+    if (tower_launches) *tower_launches = prof_drained * ((dense && persistent) ? 1 : 2 * hp.num_blocks);
     if (total_ms) *total_ms = prof_total_ms;
     if (evals) *evals = prof_drained;
     prof_drained = 0; prof_tower_ms = prof_total_ms = 0;
@@ -2182,25 +1786,14 @@ struct ResNetImpl : az_net {
       return AZ_EUNSUPPORTED;
     }
     if (hp.num_blocks < 0) { ctx->err = "ResNet: num_blocks must be >= 0"; return AZ_EINVAL; }
-    { const char* e = getenv("AZ_GENERIC_TOWER"); generic_tower = e && e[0] == '1'; }
-    { const char* e = getenv("AZ_TOWER"); dense = C4_TOWER && !generic_tower && hp.num_blocks > 0 && !(e && e[0] == 'r'); }  // AZ_TOWER=r1: round-1 kernel
+    dense = C4_TOWER && hp.num_blocks > 0;
     if (dense) { RS = W; BS = W * H; VR = W * H; KP = W * H * 32; KD = (KP + 63) / 64 * 64; }
-    { const char* e = getenv("AZ_TOWER_DEBUG"); tower_debug = e ? atoi(e) : 0; }
-    { const char* e = getenv("AZ_NO_PDL"); use_pdl = !(e && e[0] == '1'); }
     geom.row_stride = RS; geom.board_rows = BS; geom.valid_rows = VR; geom.wcols = dense ? RS : W;  // dense: every row is a cell
     for (int ky = 0; ky < 3; ky++)
       for (int kx = 0; kx < 3; kx++) geom.off[ky * 3 + kx] = (1 - ky) * (W + 1) + (1 - kx);
     smem128 = sizeof(tc::Smem<128>) + 1024;
-    smem64 = sizeof(tc::Smem<64>) + 1024;
     AZ_TRY2(set_smem(az_k_gemm_tc<128, tc::EPI_CONV1>, smem128));
     AZ_TRY2(set_smem(az_k_gemm_tc<128, tc::EPI_CONV2>, smem128));
-    AZ_TRY2(set_smem(az_k_gemm_tc<128, tc::EPI_DENSE>, smem128));
-    AZ_TRY2(set_smem(az_k_gemm_tc<64, tc::EPI_HEAD>, smem64));
-    AZ_TRY2(set_smem(az_k_gemm_tc<64, tc::EPI_DENSE>, smem64));
-    smem_2sm = sizeof(tc3::Smem);
-    static_assert(sizeof(tc3::Smem) <= 232448, "Connect-Four tower kernel exceeds the 227 KB shared-memory limit");
-    AZ_TRY2(set_smem(az_k_conv_c4_2sm<tc::EPI_CONV1>, smem_2sm));
-    AZ_TRY2(set_smem(az_k_conv_c4_2sm<tc::EPI_CONV2>, smem_2sm));
     smem_yrow = sizeof(yr::Smem);
     static_assert(sizeof(yr::Smem) <= 232448, "y-row tower kernel exceeds the 227 KB shared-memory limit");
     AZ_TRY2(set_smem(az_k_conv_yrow<tc::EPI_CONV1>, smem_yrow));
@@ -2212,9 +1805,8 @@ struct ResNetImpl : az_net {
     AZ_TRY2(set_smem(az_k_stem<G>, smem_stem));
     AZ_TRY2(set_smem(az_k_heads_dense<G>, smem128));
     AZ_TRY2(set_smem(az_k_head_conv, sizeof(hc::Smem) + 1024));
-    { const char* e = getenv("AZ_FUSED"); fused = !(e && e[0] == '0'); }
+    // AZ_TOWER=layer and AZ_LO=16 select the per-layer reference form of the Connect-Four tower (see az_k_conv_yrow)
     { const char* e = getenv("AZ_TOWER"); persistent = !(e && e[0] == 'l'); }          // AZ_TOWER=layer
-    { const char* e = getenv("AZ_TOWER_COOP"); coop_launch = !(e && e[0] == '0'); }    // AZ_TOWER_COOP=0: plain launch
     { const char* e = getenv("AZ_LO"); lo8 = !(e && e[0] == '1'); }                    // AZ_LO=16: fp16 low-order residual part
     if (cudaMalloc((void**)&d_done, 256 * sizeof(unsigned long long)) != cudaSuccess) { cudaGetLastError(); ctx->err = "cudaMalloc (tower flags) failed"; return AZ_ENOMEM; }
     cudaMemset(d_done, 0, 256 * sizeof(unsigned long long));
@@ -2246,9 +1838,9 @@ struct ResNetImpl : az_net {
     d_bstem = d_bh = d_bd = d_wv2 = d_bv2 = nullptr; d_wh = d_wd = d_wstem = nullptr;
   }
   void free_act() {
-    cudaFree(d_x32); cudaFree(d_hid); cudaFree(d_x16); cudaFree(d_t16); cudaFree(d_hp); cudaFree(d_hv); cudaFree(d_x0); cudaFree(d_logit);
+    cudaFree(d_x32); cudaFree(d_x16); cudaFree(d_t16); cudaFree(d_hp); cudaFree(d_hv);
     cudaFree(d_xl16); cudaFree(d_xl8); d_xl8 = nullptr;
-    d_x32 = d_hid = d_logit = nullptr; d_x16 = d_t16 = d_hp = d_hv = d_x0 = d_xl16 = nullptr;
+    d_x32 = nullptr; d_x16 = d_t16 = d_hp = d_hv = d_xl16 = nullptr;
   }
   ~ResNetImpl() override { free_weights(); free_act(); cudaFree(d_done); for (auto e : pev) cudaEventDestroy(e); }
 
@@ -2378,27 +1970,15 @@ struct ResNetImpl : az_net {
     free_act();
     alloc_rows = ((max_boards * BS + 127) / 128) * 128 + 128;
     alloc_boards = alloc_rows / BS;
-    const bool need_x32 = !(C4_TOWER && !generic_tower && hp.num_blocks > 0);
-    if (need_x32) AZ_TRY2(dmalloc(&d_x32, (size_t)alloc_rows * F));
+    if (!dense) AZ_TRY2(dmalloc(&d_x32, (size_t)alloc_rows * F));
     else AZ_TRY2(dmalloc(&d_xl16, (size_t)alloc_rows * F));
     AZ_TRY2(dmalloc(&d_x16, (size_t)alloc_rows * F));
     AZ_TRY2(dmalloc(&d_t16, (size_t)alloc_rows * F)); AZ_TRY2(dmalloc(&d_hp, (size_t)alloc_rows * 32));
-    AZ_TRY2(dmalloc(&d_hv, (size_t)alloc_rows * 32)); AZ_TRY2(dmalloc(&d_hid, (size_t)(max_boards + 256) * F));
-    AZ_TRY2(dmalloc(&d_x0, (size_t)alloc_rows * 64)); AZ_TRY2(dmalloc(&d_logit, (size_t)(max_boards + 256) * F));
-    AZ_TRY2(make_map_2d(ctx, &mapX0, d_x0, 64, alloc_rows, 64 * 2, tc::BK, tc::BM));
+    AZ_TRY2(dmalloc(&d_hv, (size_t)alloc_rows * 32));
     AZ_TRY2(make_map_2d(ctx, &mapHp, d_hp, (uint64_t)BS * 32, alloc_boards, (uint64_t)BS * 32 * 2, tc::BK, tc::BM));
     AZ_TRY2(make_map_2d(ctx, &mapX, d_x16, F, alloc_rows, F * 2, tc::BK, tc::BM));
     AZ_TRY2(make_map_2d(ctx, &mapT, d_t16, F, alloc_rows, F * 2, tc::BK, tc::BM));
-    AZ_TRY2(make_map_2d(ctx, &mapX2, d_x16, F, alloc_rows, F * 2, tc2::BK, tc2::AROWS));
-    AZ_TRY2(make_map_2d(ctx, &mapT2, d_t16, F, alloc_rows, F * 2, tc2::BK, tc2::AROWS));
-    AZ_TRY2(make_map_2d(ctx, &mapTo, d_t16, F, alloc_rows, F * 2, 16, 32, CU_TENSOR_MAP_SWIZZLE_32B));
-    AZ_TRY2(make_map_2d(ctx, &mapXo, d_x16, F, alloc_rows, F * 2, 16, 32, CU_TENSOR_MAP_SWIZZLE_32B));
     AZ_TRY2(make_map_2d(ctx, &mapXo64, d_x16, F, alloc_rows, F * 2, 32, 32, CU_TENSOR_MAP_SWIZZLE_64B));
-    if (!need_x32) {
-      AZ_TRY2(make_map_2d(ctx, &mapXr, d_x16, F, alloc_rows, F * 2, tc2::BK, tc2::BM));
-      AZ_TRY2(make_map_2d(ctx, &mapXLr, d_xl16, F, alloc_rows, F * 2, tc2::BK, tc2::BM));
-      AZ_TRY2(make_map_2d(ctx, &mapXLo, d_xl16, F, alloc_rows, F * 2, 16, 32, CU_TENSOR_MAP_SWIZZLE_32B));
-    }
     AZ_TRY2(make_map_2d(ctx, &mapHv, d_hv, (uint64_t)BS * 32, alloc_boards, (uint64_t)BS * 32 * 2, tc::BK, tc::BM));
     if (dense) {
       const CUtensorMapSwizzle s128 = CU_TENSOR_MAP_SWIZZLE_128B, s32 = CU_TENSOR_MAP_SWIZZLE_32B;
@@ -2425,10 +2005,9 @@ struct ResNetImpl : az_net {
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3(grid); cfg.blockDim = dim3(yr::NUM_THREADS); cfg.dynamicSmemBytes = smem_tower; cfg.stream = st;
     cudaLaunchAttribute at[2];
-    int na = 0;
-    if (use_pdl) { at[na].id = cudaLaunchAttributeProgrammaticStreamSerialization; at[na].val.programmaticStreamSerializationAllowed = 1; na++; }
-    if (coop_launch) { at[na].id = cudaLaunchAttributeCooperative; at[na].val.cooperative = 1; na++; }
-    cfg.attrs = at; cfg.numAttrs = na;
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization; at[0].val.programmaticStreamSerializationAllowed = 1;
+    at[1].id = cudaLaunchAttributeCooperative; at[1].val.cooperative = 1;
+    cfg.attrs = at; cfg.numAttrs = 2;
     const int L = 2 * hp.num_blocks;
     GemmArgs g2 = ga;
     g2.lo8 = lo8 ? 1 : 0;
@@ -2448,72 +2027,42 @@ struct ResNetImpl : az_net {
     const bool prof = profiling;
     cudaEvent_t* pe = prof ? &pev[(size_t)prof_evals * 4] : nullptr;
     if (prof) cudaEventRecord(pe[0], st);
-    const bool c4_fast = C4_TOWER && !generic_tower && two_sm && hp.num_blocks > 0;
     const int row_tiles = (max_rows * BS + tc::BM - 1) / tc::BM;
-    const int grid = std::min(row_tiles, ctx->num_sms);
     GemmArgs ga{};
-    ga.n_boards = n_rows; ga.g = geom; ga.alloc_rows = alloc_rows; ga.rows_per_board = BS; ga.debug = 0;
-    ga.gemm_k = 1; ga.kblocks = 1; ga.bias = d_bstem; ga.out16a = d_x16; ga.out32 = c4_fast ? nullptr : d_x32;
-    if (fused) {
-      launch_pdl(az_k_stem<G>, std::min(row_tiles, 2 * ctx->num_sms), st::NUM_THREADS, smem_stem, st, envs, mapWstem, mapXo64, ga, dense ? 1 : 0);
-    } else {
-      az_k_im2col<G><<<(max_rows + 3) / 4, 128, 0, st>>>(envs, n_rows, d_x0, dense ? 1 : 0);
-      launch_pdl(az_k_gemm_tc<128, tc::EPI_CONV1>, grid, tc::NUM_THREADS, smem128, st, mapX0, mapWstem, ga);
-    }
-    ga.gemm_k = 0; ga.out32 = nullptr; ga.debug = tower_debug;
+    ga.n_boards = n_rows; ga.g = geom; ga.alloc_rows = alloc_rows; ga.rows_per_board = BS;
+    ga.bias = d_bstem; ga.out16a = d_x16; ga.out32 = dense ? nullptr : d_x32;
+    launch_pdl(az_k_stem<G>, std::min(row_tiles, 2 * ctx->num_sms), st::NUM_THREADS, smem_stem, st, envs, mapWstem, mapXo64, ga, dense ? 1 : 0);
     if (prof) cudaEventRecord(pe[1], st);
-    const bool c4 = C4_TOWER && !generic_tower;  // Connect-Four geometry -> cta_group::2 kernel, otherwise the generic 9-tap kernel
-    const int grid_2sm = std::max(2, std::min(2 * ((row_tiles + 1) / 2), ctx->num_sms & ~1));
     const int grid_yr = ctx->num_sms & ~1;  // persistent: one CTA pair per SM pair, balanced unit ranges (idle pairs exit)
-    if (dense && persistent && hp.num_blocks > 0) {
+    if (dense && persistent) {
       ga.bias = d_ball;
       AZ_TRY2(launch_tower(grid_yr, st, ga));
     }
     for (int blk = 0; dense && !persistent && blk < hp.num_blocks; blk++) {
       ga.bias = d_bconv[2 * blk]; ga.res_lo = 0;
-      if (use_pdl && blk > 0) launch_pdl(az_k_conv_yrow<tc::EPI_CONV1>, grid_yr, yr::NUM_THREADS, smem_yrow, st, map4X, mapW2[2 * blk], map4To, map4XLo, map4X, map4XL, ga);
+      if (blk > 0) launch_pdl(az_k_conv_yrow<tc::EPI_CONV1>, grid_yr, yr::NUM_THREADS, smem_yrow, st, map4X, mapW2[2 * blk], map4To, map4XLo, map4X, map4XL, ga);
       else az_k_conv_yrow<tc::EPI_CONV1><<<grid_yr, yr::NUM_THREADS, smem_yrow, st>>>(map4X, mapW2[2 * blk], map4To, map4XLo, map4X, map4XL, ga);
       ga.bias = d_bconv[2 * blk + 1];
       ga.res_lo = blk > 0 ? 1 : 0;  // block 0: the residual is the fp16 stem output, no low-order part yet
-      if (use_pdl) launch_pdl(az_k_conv_yrow<tc::EPI_CONV2>, grid_yr, yr::NUM_THREADS, smem_yrow, st, map4T, mapW2[2 * blk + 1], map4Xo, map4XLo, map4X, map4XL, ga);
-      else az_k_conv_yrow<tc::EPI_CONV2><<<grid_yr, yr::NUM_THREADS, smem_yrow, st>>>(map4T, mapW2[2 * blk + 1], map4Xo, map4XLo, map4X, map4XL, ga);
+      launch_pdl(az_k_conv_yrow<tc::EPI_CONV2>, grid_yr, yr::NUM_THREADS, smem_yrow, st, map4T, mapW2[2 * blk + 1], map4Xo, map4XLo, map4X, map4XL, ga);
     }
+    const int grid = std::min(row_tiles, ctx->num_sms);
     for (int blk = 0; !dense && blk < hp.num_blocks; blk++) {
-      ga.kblocks = 18; ga.bias = d_bconv[2 * blk]; ga.resid32 = nullptr; ga.out32 = nullptr; ga.out16a = d_t16; ga.out16b = nullptr;
-      if (c4 && two_sm && use_pdl && blk > 0) launch_pdl(az_k_conv_c4_2sm<tc::EPI_CONV1>, grid_2sm, tc3::NUM_THREADS, smem_2sm, st, mapX2, mapW2[2 * blk], mapTo, mapXLo, mapXr, mapXLr, ga);
-      else if (c4 && two_sm) az_k_conv_c4_2sm<tc::EPI_CONV1><<<grid_2sm, tc3::NUM_THREADS, smem_2sm, st>>>(mapX2, mapW2[2 * blk], mapTo, mapXLo, mapXr, mapXLr, ga);
-      else az_k_gemm_tc<128, tc::EPI_CONV1><<<grid, tc::NUM_THREADS, smem128, st>>>(mapX, mapW[2 * blk], ga);
+      ga.kblocks = 18; ga.bias = d_bconv[2 * blk]; ga.out16a = d_t16;
+      az_k_gemm_tc<128, tc::EPI_CONV1><<<grid, tc::NUM_THREADS, smem128, st>>>(mapX, mapW[2 * blk], ga);
       ga.bias = d_bconv[2 * blk + 1]; ga.resid32 = d_x32; ga.out32 = d_x32; ga.out16a = d_x16;
-      ga.res_lo = blk > 0 ? 1 : 0;  // block 0: the residual is the fp16 stem output, no low-order part yet
-      if (c4 && two_sm && (tower_debug & 1)) az_k_conv_c4_2sm<tc::EPI_CONV1><<<grid_2sm, tc3::NUM_THREADS, smem_2sm, st>>>(mapT2, mapW2[2 * blk + 1], mapXo, mapXLo, mapXr, mapXLr, ga);
-      else if (c4 && two_sm && use_pdl) launch_pdl(az_k_conv_c4_2sm<tc::EPI_CONV2>, grid_2sm, tc3::NUM_THREADS, smem_2sm, st, mapT2, mapW2[2 * blk + 1], mapXo, mapXLo, mapXr, mapXLr, ga);
-      else if (c4 && two_sm) az_k_conv_c4_2sm<tc::EPI_CONV2><<<grid_2sm, tc3::NUM_THREADS, smem_2sm, st>>>(mapT2, mapW2[2 * blk + 1], mapXo, mapXLo, mapXr, mapXLr, ga);
-      else az_k_gemm_tc<128, tc::EPI_CONV2><<<grid, tc::NUM_THREADS, smem128, st>>>(mapT, mapW[2 * blk + 1], ga);
+      az_k_gemm_tc<128, tc::EPI_CONV2><<<grid, tc::NUM_THREADS, smem128, st>>>(mapT, mapW[2 * blk + 1], ga);
     }
     if (prof) cudaEventRecord(pe[2], st);
-    // heads: 1x1 convs (both heads, N = 64), value dense (K = KD), finalize
-    ga.g.off[0] = 0;  // 1x1 conv: single centre tap
-    ga.debug = 0;
-    ga.kblocks = 2; ga.bias = d_bh; ga.resid32 = nullptr; ga.out32 = nullptr; ga.out16a = d_hp; ga.out16b = d_hv;
-    if (fused) launch_pdl(az_k_head_conv, std::min(row_tiles, 2 * ctx->num_sms), hc::NUM_THREADS, sizeof(hc::Smem) + 1024, st, mapX, mapWh, ga);
-    else launch_pdl(az_k_gemm_tc<64, tc::EPI_HEAD>, grid, tc::NUM_THREADS, smem64, st, mapX, mapWh, ga);
-    GemmArgs gd{};
-    gd.n_boards = n_rows; gd.g = geom; gd.kblocks = KD / 64; gd.gemm_k = 1; gd.rows_per_board = 1; gd.alloc_rows = max_rows + 256;
-    gd.bias = d_bd; gd.out32 = d_hid;
+    // heads: both 1x1 convs (N = 64), then the value / policy dense layers and outputs
+    ga.bias = d_bh; ga.out16a = d_hp; ga.out16b = d_hv;
+    launch_pdl(az_k_head_conv, std::min(row_tiles, 2 * ctx->num_sms), hc::NUM_THREADS, sizeof(hc::Smem) + 1024, st, mapX, mapWh, ga);
     const int board_tiles = (max_rows + tc::BM - 1) / tc::BM;
-    if (fused) {
-      HeadArgs ha{n_rows, KD / 64, d_bd, d_wv2, d_bv2, d_bpol, dbg_logit, dbg_vpre};
-      const int hgrid = 2 * std::max(1, std::min(board_tiles, ctx->num_sms / 2));
-      launch_pdl(az_k_heads_dense<G>, hgrid, tc::NUM_THREADS, smem128, st, mapHv, mapWd, mapHp, mapWpol, ha, envs, P, V, Pinv);
-    } else {
-      launch_pdl(az_k_gemm_tc<128, tc::EPI_DENSE>, std::min(board_tiles, ctx->num_sms), tc::NUM_THREADS, smem128, st, mapHv, mapWd, gd);
-      gd.bias = d_bpol; gd.out32 = d_logit; gd.no_relu = 1;   // policy dense: logits[b][0..A) = Wp . hp + b
-      launch_pdl(az_k_gemm_tc<64, tc::EPI_DENSE>, std::min(board_tiles, ctx->num_sms), tc::NUM_THREADS, smem64, st, mapHp, mapWpol, gd);
-      FinalArgs fa{d_logit, d_hid, d_wv2, d_bv2, dbg_logit, dbg_vpre};
-      az_k_finalize<G><<<(max_rows * 8 + 255) / 256, 256, 0, st>>>(envs, n_rows, fa, P, V, Pinv);
-    }
+    HeadArgs ha{n_rows, KD / 64, d_bd, d_wv2, d_bv2, d_bpol, dbg_logit, dbg_vpre};
+    const int hgrid = 2 * std::max(1, std::min(board_tiles, ctx->num_sms / 2));
+    launch_pdl(az_k_heads_dense<G>, hgrid, tc::NUM_THREADS, smem128, st, mapHv, mapWd, mapHp, mapWpol, ha, envs, P, V, Pinv);
     if (prof) { cudaEventRecord(pe[3], st); prof_evals++; }
-    ctx->launches += (fused ? 3 : 6) + ((dense && persistent && hp.num_blocks > 0) ? 1 : 2 * hp.num_blocks);
+    ctx->launches += 3 + ((dense && persistent) ? 1 : 2 * hp.num_blocks);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) { ctx->err = std::string("network launch: ") + cudaGetErrorString(e); return AZ_ECUDA; }
     return AZ_OK;

@@ -28,13 +28,13 @@ def unit_range(n_boards, pair, npairs=NPAIRS):
     return U * pair // npairs, U * (pair + 1) // npairs
 
 
-def segments(u0, u1, natural=False):
+def segments(u0, u1):
     """Processing order of a pair's segments: (g, j_lo, j_hi) -- tw::segment()."""
     nseg = (u1 - 1) // H - u0 // H + 1
     out = []
     for k in range(nseg):
         i = k
-        if not natural and nseg >= 2 and u1 % H != 0:   # a range that ends on a group boundary has no reader above
+        if nseg >= 2 and u1 % H != 0:   # a range that ends on a group boundary has no reader above
             i = nseg - 1 if k == 0 else k - 1
         g = u0 // H + i
         j_lo = u0 - g * H if i == 0 else 0
@@ -84,7 +84,7 @@ class Graph:
         return anc
 
 
-def build(n_boards, num_layers, natural=False, resources=True, drop=()):
+def build(n_boards, num_layers, resources=True, drop=()):
     """Events: ('L', p, l, g, y) input row y of group g requested by the producer; ('C', p, l, g, y) its stages consumed by the MMAs;
     ('A', p, l, u) accumulator of output row u complete; ('E', p, l, u) epilogue of u (the TMA stores are issued: the WRITE);
     ('S', p, l, u) stores complete and published (stored[] += 1, and the pair's counters if u is its first / last row);
@@ -102,7 +102,7 @@ def build(n_boards, num_layers, natural=False, resources=True, drop=()):
         q_hi = upper[p] if u1 % H != 0 else None
         prev_load = prev_cons = prev_epi = prev_store = None
         for l in range(num_layers):
-            segs = segments(u0, u1, natural)
+            segs = segments(u0, u1)
             units = [g * H + j for (g, j_lo, j_hi) in segs for j in range(j_lo, j_hi)]
             order_check.append((p, l, units))
             if l > 0 and "wfree" not in drop:
@@ -152,15 +152,15 @@ def build(n_boards, num_layers, natural=False, resources=True, drop=()):
     return G, pairs, rng, reads, order_check
 
 
-def check(n_boards, num_layers=4, natural=False, drop=()):
+def check(n_boards, num_layers=4, drop=()):
     # 1. no deadlock under the tightest resource limits
-    G, pairs, rng, reads, order_check = build(n_boards, num_layers, natural, resources=True, drop=drop)
+    G, pairs, rng, reads, order_check = build(n_boards, num_layers, resources=True, drop=drop)
     assert G.topo() is not None, "cyclic wait graph (deadlock) at %d boards" % n_boards
     # 2. every unit exactly once, all roles in the same order (the three device loops share tw::segment)
     for p, l, units in order_check:
         assert sorted(units) == list(range(*rng[p])), (p, l)
     # 3. hazards, from protocol edges only
-    G, pairs, rng, reads, _ = build(n_boards, num_layers, natural, resources=False, drop=drop)
+    G, pairs, rng, reads, _ = build(n_boards, num_layers, resources=False, drop=drop)
     anc = G.ancestors()
     owner = {}
     for p in pairs:
@@ -184,13 +184,11 @@ def check(n_boards, num_layers=4, natural=False, drop=()):
     return len(pairs), n_raw, n_war
 
 
-@pytest.mark.parametrize("natural", [False, True])
-def test_tower_protocol_small_and_odd_sizes(natural):
-    """Every board count up to 20 groups = 640 boards (one unit per pair, neighbours without work, ranges inside one group, ...);
-    the range-order variant of the A/B switch (AZ_TOWER_DEBUG=16) on every 7th."""
+def test_tower_protocol_small_and_odd_sizes():
+    """Every board count up to 20 groups = 640 boards (one unit per pair, neighbours without work, ranges inside one group, ...)."""
     seen_pairs = set()
-    for n in list(range(1, 32 * 20 + 1, 1 if not natural else 7)) + [1, 31, 32, 33, 63, 64, 65, 395, 396, 397]:
-        npairs, n_raw, n_war = check(n, natural=natural)
+    for n in list(range(1, 32 * 20 + 1)) + [1, 31, 32, 33, 63, 64, 65, 395, 396, 397]:
+        npairs, n_raw, n_war = check(n)
         seen_pairs.add(npairs)
         assert n_raw > 0
     assert 6 in seen_pairs and 74 in seen_pairs      # one group = six pairs with one unit each ... all 74 pairs busy
